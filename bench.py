@@ -7,12 +7,20 @@ conditioner, K=10 knots, batch 16384 per GPU), on N GPUs of one node.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the CPU arm: the unmodified reference on the host cores
+    python bench.py --steps 10 --warmup 3 --dump-outputs DIR   # also write the last timed step's results
 
 One "step" = one pass of the hot path over one synthetic batch: NormalPrior draw with
 log-density -> four checkerboard RQ-spline coupling steps (conditioner + spline +
 log|det J|) -> phi^4 action, i.e. `model.posterior.sample__(B)`.  Ranks are independent
 (batch sharding, no data-path collective): weak scaling, `value` = all ranks' samples
 divided by the slowest rank's device time.
+
+--dump-outputs DIR writes what the last timed step returned on rank 0, as .npy files (float32, or
+float64 where the path returns that):
+DIR/logq.npy and DIR/logp.npy (B values each) and DIR/y_sample.npy, the transformed fields y of a
+fixed, seeded sample of 2048 of the B samples (32 MB; all of them when B <= 2048).  The model
+weights and the prior draws are seeded, so two runs with the same arguments see the same inputs
+and two builds can be compared output for output.
 
 The JSON line carries, besides the base contract:
   roofline     : the dominant kernel (the fused coupling step), algorithmic bytes (SURVEY 8d:
@@ -75,7 +83,14 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip train_step / mcmc / configs")
     ap.add_argument("--train-batch", type=int, default=None, help="samples per GPU of the training step (default: --batch)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's logq, logp and a fixed sample of y to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl b200)")
+    return a
 
 
 # --------------------------------------------------------------------------- CPU arm
@@ -263,6 +278,21 @@ def _timed_loop(torch, dist, world, barrier, fn, steps, warmup):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = t.item()
     return ms
+
+
+DUMP_Y_ROWS = 2048
+
+
+def dump_outputs(path, y, logq, logp):
+    """--dump-outputs: the results of one step as DIR/<name>.npy (see the module docstring)."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    B = y.shape[0]
+    rows = np.arange(B) if B <= DUMP_Y_ROWS else np.sort(np.random.default_rng(0).choice(B, DUMP_Y_ROWS, replace=False))
+    arrays = {"logq": logq, "logp": logp, "y_sample": y[torch.as_tensor(rows, device=y.device)]}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 def _prepare_training(torch, model, world, rank, batch):
@@ -500,6 +530,8 @@ def run_b200(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = t.item()
     value = world * B * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y, logq, logp)
 
     # ---- end to end with host buffers ---------------------------------------------------
     e2e = None

@@ -74,23 +74,42 @@ def test_library_is_sm100a_only():
 
 
 # ------------------------------------------------------------------ no CPU fallback
-def test_hot_path_refuses_cpu_tensors():
-    if torch.cuda.is_available():
-        pytest.skip("GPU present: covered by the gpu tests")
-    act = ScalarPhi4Action(m_sq=-1.2, lambd=0.5)
-    with pytest.raises(RuntimeError, match="CUDA"):
-        act(torch.zeros(2, 4, 4))
-    prior = NormalPrior(shape=(4, 4))
-    with pytest.raises(RuntimeError, match="CUDA"):
-        prior.sample(2)
-    with pytest.raises(RuntimeError, match="CUDA"):
-        prior.log_prob(torch.zeros(2, 4, 4))
-    mask = EvenOddMask(shape=(4, 4))
-    cpl = AffineCoupling_([ConvAct(1, 2, 3, hidden_sizes=[4], acts=['tanh', None])], mask=mask)
-    with pytest.raises(RuntimeError, match="CUDA"):
-        cpl(torch.zeros(2, 4, 4))
-    with pytest.raises(RuntimeError, match="CUDA"):
-        DistConvertor_(5, symmetric=True)(torch.zeros(3, 1))
+_NO_CUDA = r'''
+import sys
+sys.path.insert(0, {root!r})
+import pytest, torch
+assert not torch.cuda.is_available()
+from normflow__b200.action import ScalarPhi4Action
+from normflow__b200.mask import EvenOddMask
+from normflow__b200.nn import AffineCoupling_, ConvAct, DistConvertor_
+from normflow__b200.prior import NormalPrior
+
+act = ScalarPhi4Action(m_sq=-1.2, lambd=0.5)
+with pytest.raises(RuntimeError, match="CUDA"):
+    act(torch.zeros(2, 4, 4))
+prior = NormalPrior(shape=(4, 4))
+with pytest.raises(RuntimeError, match="CUDA"):
+    prior.sample(2)
+with pytest.raises(RuntimeError, match="CUDA"):
+    prior.log_prob(torch.zeros(2, 4, 4))
+mask = EvenOddMask(shape=(4, 4))
+cpl = AffineCoupling_([ConvAct(1, 2, 3, hidden_sizes=[4], acts=['tanh', None])], mask=mask)
+with pytest.raises(RuntimeError, match="CUDA"):
+    cpl(torch.zeros(2, 4, 4))
+with pytest.raises(RuntimeError, match="CUDA"):
+    DistConvertor_(5, symmetric=True)(torch.zeros(3, 1))
+print("refused")
+'''
+
+
+def test_hot_path_refuses_cpu_tensors(tmp_path):
+    """Without a visible CUDA device the package keeps its objects on the CPU, and every kernel entry
+    refuses them.  Runs in a child process with the GPUs hidden, so that it checks this on any machine."""
+    script = tmp_path / "no_cuda.py"
+    script.write_text(_NO_CUDA.format(root=ROOT))
+    r = subprocess.run([sys.executable, str(script)], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=240)
+    assert r.returncode == 0 and "refused" in r.stdout, r.stdout
 
 
 # ------------------------------------------------------------------ masks (bit-exact)
