@@ -7,6 +7,8 @@
 //   x  strip : rows r0-3 .. r0+rows+2   fp32   [rows+6][WS]
 //   h1 strip : rows r0-2 .. r0+rows+1   fp16 hi/lo planes of 16-byte records (8 channels)
 //   h2 strip : rows r0-1 .. r0+rows     the same, split by the parity of the linear index
+// A strip that continues a sample copies its first h2 rows (0, 1) and the h1 rows they need (2, 3)
+// from the bottom of the previous strip instead of recomputing them (tc_carry).
 //
 //   compute warps                                   MMA warp
 //   -------------                                   --------
@@ -14,7 +16,7 @@
 //   P1: h1 = tanh(conv1(x frozen))  -> arrive H1    sync H1: layer-2 tiles (9 MMAs each, N = 16),
 //   E2: per tile wait m2[j]; TMEM -> bias, tanh,             commit m2[j] per tile
 //       split -> h2                 -> arrive H2    sync H2: layer-3 tiles on ACTIVE sites
-//   E3: per tile wait m3[k]; TMEM -> spline/affine           (9 MMAs, N = 2 NP), commit m3[k]
+//   E3: per tile wait m3[k]; TMEM -> spline/affine           (9 MMAs, N = N3), commit m3[k]
 //       -> y into the x strip       |barC|
 //   copy the strip's rows to y      |barC|
 
@@ -69,7 +71,8 @@ __device__ __forceinline__ void make_records(const float (&v)[8], uint4& hi, uin
 template <int KIND, int K, int INV, bool SAVE>
 __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs a) {
     constexpr int P = KIND == 0 ? 2 : 3 * K - 2;
-    constexpr int NP = TcShape<P>::NP, N3 = TcShape<P>::N3;
+    using Shape = TcShape<P>;
+    constexpr int N3 = Shape::N3;
     extern __shared__ __align__(128) uint8_t smem[];
     const TcGeom& g = a.g;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -80,7 +83,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
     uint8_t* h2 = smem + g.off_h2 + kTcGuard * 16;            // record 0 of parity 0, hi plane
     __half* B2 = reinterpret_cast<__half*>(smem + g.off_b2);  // [tap][kgroup][16][8]
     __half* B3 = reinterpret_cast<__half*>(smem + g.off_b3);  // [tap][kgroup][N3][8]
-    float* w1s = reinterpret_cast<float*>(smem + g.off_w1);   // [tap][8] | b1[8] | b2[8] | b3[NP]
+    float* w1s = reinterpret_cast<float*>(smem + g.off_w1);   // [tap][8] | b1[8] | b2[8] | b3[P]
     float* b1s = w1s + 72;                                    // layer-1 weights and b1, b2 are stored times
     float* b2s = b1s + 8;                                     // 2 log2(e): the tanh argument comes out scaled
     float* b3s = b2s + 8;
@@ -98,19 +101,22 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
         B2[((t * 2 + 0) * 16 + n) * 8 + ci] = val;
         B2[((t * 2 + 1) * 16 + n) * 8 + ci] = val;
     }
-    for (int e = tid; e < 9 * N3 * 8; e += kTcThreads) {                 // layer 3: N = [NP hi | NP lo]
+    for (int e = tid; e < 9 * N3 * 8; e += kTcThreads) {                 // layer 3: N = [8 hi | 8 lo] per group
         const int ci = e & 7, n = (e >> 3) % N3, t = (e >> 3) / N3;
-        const int p = n < NP ? n : n - NP;
+        const int grp = n >> 4, w16 = n & 15;
+        const int gs = P - 8 * grp < 8 ? P - 8 * grp : 8;                // channels of this group (<= 0: padding)
+        const bool is_lo = w16 >= gs;
+        const int p = 8 * grp + (is_lo ? w16 - gs : w16);
         __half val = __float2half_rn(0.f);
-        if (p < P) {
+        if (w16 < 2 * gs) {
             const float w = NFK_LDG(a.w3 + (p * 8 + ci) * 9 + t);
             const __half hi = __float2half_rn(w);
-            val = n < NP ? hi : __float2half_rn((w - __half2float(hi)) * kLoScale);
+            val = is_lo ? __float2half_rn((w - __half2float(hi)) * kLoScale) : hi;
         }
         B3[((t * 2 + 0) * N3 + n) * 8 + ci] = val;
         B3[((t * 2 + 1) * N3 + n) * 8 + ci] = val;
     }
-    for (int e = tid; e < 72 + 8 + 8 + NP; e += kTcThreads) {
+    for (int e = tid; e < 72 + 8 + 8 + P; e += kTcThreads) {
         float v;
         if (e < 72) v = kTwoLog2e * NFK_LDG(a.w1 + (e & 7) * 9 + (e >> 3));          // w1s[tap][co]
         else if (e < 80) v = a.b1 ? kTwoLog2e * NFK_LDG(a.b1 + e - 72) : 0.f;
@@ -155,9 +161,10 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
         };
         for (Unit u{blockIdx.x, 0}; u.b < a.B; u = next_unit(u)) {
             const int r0 = u.r0, rows = L0 - r0 < Rr ? L0 - r0 : Rr;
-            const int t2 = tc_tiles2(rows, WS), t3 = tc_tiles3(rows, WS, L1);
+            const int c2 = tc_carry(r0);
+            const int t2 = tc_tiles2(rows, WS, c2), t3 = tc_tiles3(rows, WS, L1);
             const int plin = (g.active_val - 1 + g.mask_parity - r0) & 1;
-            // ---- layer 2: out record i2 = 128 j + m reads h1 records i2 + WS + dr WS + dc
+            // ---- layer 2: out record i2 = c2 WS + 128 j + m reads h1 records i2 + WS + dr WS + dc
             stamp(0);
             tc::bar_sync(kBarH1, kTcThreads);
             tc::fence_after_sync();
@@ -167,7 +174,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
 #pragma unroll
                     for (int t = 0; t < 9; ++t) {
                         const int delta = (t / 3 - 1) * WS + (t % 3 - 1);
-                        tc::mma_f16(tmem + j * 16, tc::desc_advance(a1_desc, j * 128 + WS + delta),
+                        tc::mma_f16(tmem + j * 16, tc::desc_advance(a1_desc, j * 128 + (c2 + 1) * WS + delta),
                                     tc::desc_advance(b2_desc, t * 2 * 16), idesc2, t > 0);
                     }
                     tc::mma_commit(tc::smem_u32(bars + j));
@@ -321,9 +328,9 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
                         *reinterpret_cast<uint4*>(dw) = hi;
                         *reinterpret_cast<uint4*>(dw + g.h1_comp_bytes) = lo;
                     }
-                    if (SAVE) {                                           // rows of the strip proper, not its halo
+                    if (SAVE) {   // rows of the strip proper, and the two the next strip takes over (tc_carry)
                         const int j1 = 2 * jp[z] + s;
-                        if (j1 >= 2 && j1 < rows + 2) {
+                        if (j1 >= 2 && r0 - 2 + j1 < L0) {
                             float* dsth = a.save_h1 + (b * 8 * L0 + (r0 - 2 + j1)) * (long long)L1 + c;
 #pragma unroll
                             for (int co = 0; co < 8; ++co)
@@ -336,7 +343,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
         auto layer1 = [&](const Unit& u, const float* xbuf) {
             const int r0 = u.r0, rows = L0 - r0 < Rr ? L0 - r0 : Rr;
             const int npair = (rows + 5) >> 1, items = npair * L1;
-            int it0 = tid;
+            int it0 = tid + tc_carry(r0) * L1;                        // first pair: h1 rows 2 carry, 2 carry + 1
             for (; it0 + kTcComputeThreads < items; it0 += 2 * kTcComputeThreads)
                 layer1_items(std::integral_constant<int, 2>{}, it0, u.b, r0, rows, xbuf);
             if (it0 < items) layer1_items(std::integral_constant<int, 1>{}, it0, u.b, r0, rows, xbuf);
@@ -352,7 +359,8 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
         // ---- E2: accumulators of layer 2 -> h2 records
         auto epilogue2 = [&](const Unit& u) {
             const int rows = L0 - u.r0 < Rr ? L0 - u.r0 : Rr;
-            const int t2 = tc_tiles2(rows, WS);
+            const int c2 = tc_carry(u.r0);
+            const int t2 = tc_tiles2(rows, WS, c2);
             float bv[8];
             load_w8(b2s, bv);
             for (int j = set; j < t2; j += kTcSets) {
@@ -361,7 +369,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
                 float acc[16];
                 tc::tmem_ld16(lane_addr + j * 16, acc);
                 tc::tmem_ld_wait();
-                const int i2 = j * 128 + q * 32 + lane;
+                const int i2 = c2 * WS + j * 128 + q * 32 + lane;
                 const int j2 = tc_div(i2, g.magic_ws), slot = i2 - j2 * WS;
                 if (j2 < rows + 2 && slot >= 1 && slot <= L1) {
                     float v[8];
@@ -379,7 +387,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
                         *reinterpret_cast<uint4*>(dw) = hi;
                         *reinterpret_cast<uint4*>(dw + g.h2_comp_bytes) = lo;
                     }
-                    if (SAVE && j2 >= 1 && j2 <= rows) {
+                    if (SAVE && j2 >= 1 && u.r0 - 1 + j2 < L0) {     // row rows + 1: the next strip's row 1
                         float* dsth = a.save_h2 + (u.b * 8 * L0 + (u.r0 - 1 + j2)) * (long long)L1 + slot - 1;
 #pragma unroll
                         for (int c = 0; c < 8; ++c) dsth[(long long)c * L0 * L1] = v[c];
@@ -410,15 +418,24 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
             for (int k = set; k < t3; k += kTcSets) {
                 tile_wait(bars + 16 + k, (ph3 >> k) & 1u);
                 ph3 ^= 1u << k;
-                float prm[NP];
+                float prm[P];
 #pragma unroll
-                for (int ch = 0; ch < NP / 16; ++ch) {
-                    float hi[16], lo[16];
-                    tc::tmem_ld16(lane_addr + k * N3 + ch * 16, hi);
-                    tc::tmem_ld16(lane_addr + k * N3 + NP + ch * 16, lo);
+                for (int grp = 0; grp < Shape::kFull; ++grp) {
+                    float v[16];                                  // [8 hi | 8 lo]
+                    tc::tmem_ld16(lane_addr + k * N3 + grp * 16, v);
                     tc::tmem_ld_wait();
 #pragma unroll
-                    for (int c = 0; c < 16; ++c) prm[ch * 16 + c] = fmaf(lo[c], 1.f / kLoScale, hi[c]);
+                    for (int c = 0; c < 8; ++c) prm[grp * 8 + c] = fmaf(v[8 + c], 1.f / kLoScale, v[c]);
+                }
+                if constexpr (Shape::kTail > 0) {                 // [kTail hi | kTail lo]
+                    constexpr int kT = Shape::kTail;
+                    float v[2 * kT <= 8 ? 8 : 16];
+                    const uint32_t col = lane_addr + k * N3 + Shape::kFull * 16;
+                    if constexpr (2 * kT <= 8) tc::tmem_ld8(col, v);
+                    else tc::tmem_ld16(col, v);
+                    tc::tmem_ld_wait();
+#pragma unroll
+                    for (int c = 0; c < kT; ++c) prm[Shape::kFull * 8 + c] = fmaf(v[kT + c], 1.f / kLoScale, v[c]);
                 }
                 if (has_b3) {
 #pragma unroll
@@ -440,7 +457,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
                         if (!INV) { out = fmaf(xv, fast_ex2(-sc * kInvLn2), t); l = -sc; }
                         else { out = (xv - t) * fast_ex2(sc * kInvLn2); l = sc; }
                     } else {
-                        tc_rqs<K, INV, NP>(prm, a.cfg, xv, out, l);
+                        tc_rqs<K, INV, P>(prm, a.cfg, xv, out, l);
                     }
                     *px = out;
                     lsum += l;
@@ -448,6 +465,27 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
                 release_if_clear(k + kTcSets);
             }
             return lsum;
+        };
+
+        // tc_carry: h1 rows rows + 2, rows + 3 (hi and lo planes) -> rows 2, 3 for the next strip
+        auto carry_h1 = [&](int rows) {
+            const int n = 2 * WS;
+            for (int e = tid; e < 2 * n; e += kTcComputeThreads) {
+                const int plane = e >= n, i = e - plane * n;
+                uint8_t* dst = h1 + plane * g.h1_comp_bytes + (2 * WS + i) * 16;
+                *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(dst + rows * WS * 16);
+            }
+        };
+        // tc_carry: h2 rows rows, rows + 1 -> rows 0, 1 (the shift moves a record to the other parity
+        // plane when rows is odd)
+        auto carry_h2 = [&](int rows) {
+            const int n = 2 * WS;
+            for (int e = tid; e < 2 * n; e += kTcComputeThreads) {
+                const int plane = e >= n, i = e - plane * n, is = rows * WS + i;
+                uint8_t* h2c = h2 + plane * g.h2_comp_bytes;
+                *reinterpret_cast<uint4*>(h2c + (i & 1) * g.h2_par_bytes + (i >> 1) * 16) =
+                    *reinterpret_cast<const uint4*>(h2c + (is & 1) * g.h2_par_bytes + (is >> 1) * 16);
+            }
         };
 
         // Software pipeline over units: while the tensor core runs layer 3 of unit i, the compute
@@ -471,6 +509,8 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
         while (cur.b < a.B) {
             const Unit nxt = next_unit(cur);
             const bool has_next = nxt.b < a.B;
+            const bool carry = has_next && tc_carry(nxt.r0) > 0;
+            const int rows = L0 - cur.r0 < Rr ? L0 - cur.r0 : Rr;
             float* xcur = xs + buf * xs_stride;
             float* xnext = xs + (buf ^ 1) * xs_stride;
             stamp(0);
@@ -484,18 +524,22 @@ __global__ void __launch_bounds__(kTcThreads, 2) fused2d_tc_kernel(const TcArgs 
             tc::bar_sync(kBarCompute, kTcComputeThreads);             // x of `nxt` visible; every layer-2 tile of `cur` consumed
             stamp(2);
             int next_cols = 0;
+            if (carry) {
+                carry_h1(rows);
+                tc::bar_sync(kBarCompute, kTcComputeThreads);         // before layer 1 of `nxt` overwrites the source rows
+            }
             if (has_next) {
                 layer1(nxt, xnext);                                   // overlaps layer 3 of `cur` on the tensor core
                 tc::fence_async_smem();                               // h1 of `nxt` visible to the tensor core
                 const int nrows = L0 - nxt.r0 < Rr ? L0 - nxt.r0 : Rr;
-                next_cols = 16 * tc_tiles2(nrows, WS);
+                next_cols = 16 * tc_tiles2(nrows, WS, tc_carry(nxt.r0));
             }
             stamp(3);
             lacc += epilogue3(cur, xcur, next_cols);                  // releases layer 2 of `nxt` on the way
             stamp(4);
             tc::bar_sync(kBarCompute, kTcComputeThreads);             // y of the strip complete in xcur
+            if (carry) carry_h2(rows);                               // every layer-3 MMA of `cur` has completed
             {   // the strip's rows (active: transformed, frozen: copied) -> y, one warp per row
-                const int rows = L0 - cur.r0 < Rr ? L0 - cur.r0 : Rr;
                 float* yb = a.y + cur.b * (long long)L0 * L1;
                 for (int j = warp; j < rows; j += kTcComputeWarps) {
                     const float* src = xcur + (j + 3) * WS + 1;

@@ -9,7 +9,8 @@
 //     hi = fp16(v), lo = fp16(v - hi) (weights: lo scaled by 2^11 to stay normal).  One
 //     kind::f16 MMA has K = 16 = [8 channels of hi | 8 channels of lo] of the activations
 //     against [w_hi ; w_hi] in accumulator columns [0, N) and [w_lo ; w_lo] in columns
-//     [N, 2N): acc = (a_hi + a_lo) w_hi + 2^-11 (a_hi + a_lo) w_lo' -- 22 significant bits
+//     [N, 2N) (layer 3 interleaves the two per group of 8 channels, TcShape):
+//     acc = (a_hi + a_lo) w_hi + 2^-11 (a_hi + a_lo) w_lo' -- 22 significant bits
 //     per factor, fp32 accumulation in TMEM.  The 1e-5 parity contract rules out plain
 //     fp16 / bf16 / tf32 (SURVEY 7, hard part 1); this split costs ONE MMA per tap.
 //   * a strip of the lattice lives in shared memory as 16-byte records (one site = 8 fp16
@@ -72,8 +73,12 @@ struct TcGeom {
 __device__ __forceinline__ int tc_div(int n, uint32_t magic) { return (int)__umulhi((uint32_t)n, magic); }
 
 NFK_HD int tc_div_up(int a, int b) { return (a + b - 1) / b; }
+// A strip that continues a sample (r0 > 0) takes over from the previous strip of that sample the
+// rows both need: h2 rows 0, 1 and h1 rows 2, 3 (h1 rows 0, 1 are then read by no output).  Its
+// layer 2 starts at h2 row `carry` and its layer 1 at h1 row 2 `carry`.
+NFK_HD int tc_carry(int r0) { return r0 > 0 ? 2 : 0; }
 // tiles of layer 2 / layer 3 for a strip with `rows` output rows
-NFK_HD int tc_tiles2(int rows, int WS) { return tc_div_up((rows + 2) * WS, 128); }
+NFK_HD int tc_tiles2(int rows, int WS, int carry) { return tc_div_up((rows + 2 - carry) * WS, 128); }
 NFK_HD int tc_cbase(int WS) { return (WS + 1) >> 1; }
 NFK_HD int tc_tiles3(int rows, int WS, int L1) {
     // linear indices of the output sites in the h2 strip: rows 1..rows, slots 1..L1
@@ -81,10 +86,15 @@ NFK_HD int tc_tiles3(int rows, int WS, int L1) {
     return tc_div_up((s_max >> 1) - tc_cbase(WS) + 1, 128);
 }
 
+// Layer-3 accumulator columns, packed by groups of 8 output channels: group g holds
+// [hi of its gs channels | lo of the same], gs = min(8, P - 8 g), at columns 16 g ... 16 g + 2 gs.
+// One 16-column TMEM load (8 for a tail of <= 4 channels) then carries both halves of its
+// channels: the epilogue loads 2P columns rounded up to 8, not 2 x (P rounded up to 16).
 template <int P>
 struct TcShape {
-    static constexpr int NP = (P + 15) / 16 * 16;   // output channels padded to the MMA N granularity
-    static constexpr int N3 = 2 * NP;               // [hi block | lo block]
+    static constexpr int kFull = P / 8, kTail = P % 8;      // full groups, channels of the last group
+    static constexpr int kCols = 16 * kFull + 2 * kTail;    // accumulator columns in use
+    static constexpr int N3 = (kCols + 15) / 16 * 16;       // the MMA's N (multiple of 16 at M = 128)
 };
 
 // Fills the geometry for a given R; returns false when it does not fit one CTA's budget.
@@ -92,13 +102,14 @@ template <int P>
 inline bool tc_plan(TcGeom& g, int R, uint32_t smem_budget) {
     const int WS = g.WS;
     g.R = R;
-    const int t2 = tc_tiles2(R, WS), t3 = tc_tiles3(R, WS, g.L1);
+    const int t2 = tc_tiles2(R, WS, 0), t3 = tc_tiles3(R, WS, g.L1);
     if (t2 > 16 || t2 * 16 > kTcTmemCols || t3 > 8 || t3 * TcShape<P>::N3 > kTcTmemCols) return false;
     if ((R + 6) * WS > 6 * kTcComputeThreads) return false;                 // x strip staged in 6 registers per thread
     auto align = [](uint32_t v) { return (v + 127u) & ~127u; };
     uint32_t off = 0;
     g.off_xs = off; off = align(off + 2u * (uint32_t)(R + 7) * WS * 4); // two strips (+ 1 row: P1 pairs may peek past the end)
-    const int n1 = t2 * 128 + 2 * WS + 2;                                   // records an M2 tile may touch
+    const int e2 = t2 * 128 > 2 * WS + tc_tiles2(R, WS, 2) * 128 ? t2 * 128 : 2 * WS + tc_tiles2(R, WS, 2) * 128;
+    const int n1 = e2 + 2 * WS + 2;                                         // records an M2 tile may touch
     g.h1_comp_bytes = align((uint32_t)(kTcGuard + n1) * 16);
     g.off_h1 = off; off += 2 * g.h1_comp_bytes;
     int n2 = tc_cbase(WS) + t3 * 128 + (WS + 1) / 2 + 2;                    // per parity plane
@@ -109,7 +120,7 @@ inline bool tc_plan(TcGeom& g, int R, uint32_t smem_budget) {
     g.off_h2 = off; off += 2 * g.h2_par_bytes;
     g.off_b2 = off; off = align(off + 9 * 2 * 16 * 16);
     g.off_b3 = off; off = align(off + 9 * 2 * TcShape<P>::N3 * 16);
-    g.off_w1 = off; off = align(off + (72 + 8 + 8 + TcShape<P>::NP) * 4);
+    g.off_w1 = off; off = align(off + (72 + 8 + 8 + P) * 4);
     g.off_bar = off; off = align(off + 24 * 8 + 64);
     g.smem_bytes = off;
     return g.smem_bytes <= smem_budget;
@@ -123,7 +134,7 @@ inline float tc_cost_per_row(int L0, int L1, int WS, int R) {
     float total = 0.f;
     for (int r0 = 0; r0 < L0; r0 += R) {
         const int rows = L0 - r0 < R ? L0 - r0 : R;
-        total += tc_tiles2(rows, WS) * c2 + tc_tiles3(rows, WS, L1) * c3 + 600.f;   // + per-strip sync overhead
+        total += tc_tiles2(rows, WS, tc_carry(r0)) * c2 + tc_tiles3(rows, WS, L1) * c3 + 600.f;   // + per-strip sync overhead
     }
     return total / L0;
 }
